@@ -142,6 +142,71 @@ def _key_is(col, slab_ptr, slab_len, literal: bytes):
     return mask
 
 
+DUMP_VALUES_MAX = 1 << 19  # per dumped array: 4 MB of float64, so the eleven arrays stay under DUMP_BYTES_MAX
+DUMP_BYTES_MAX = 64 << 20
+DUMP_SEED = 0
+
+
+class _DeviceBytes:
+    """`nbytes` bytes at a device address, readable by torch through the CUDA array interface."""
+
+    def __init__(self, addr: int, nbytes: int):
+        self.__cuda_array_interface__ = {"shape": (nbytes,), "typestr": "|u1", "data": (addr, False), "version": 2}
+
+
+def device_changeset(torch, cs):
+    """Host copies of the arrays of a device-resident gar_changeset (what gar_diff_device hands its caller), under the names of
+    abi.ChangeSet.  Call it before the next diff or load on the engine: the pointers are only valid until then."""
+    import numpy as np
+    from types import SimpleNamespace
+    abi = importlib.import_module("aws-global-accelerator-controller_b200.abi")
+
+    def pull(ptr, n, dtype):
+        nbytes = int(n) * np.dtype(dtype).itemsize
+        if nbytes == 0:
+            return np.zeros(0, dtype=dtype)
+        raw = torch.as_tensor(_DeviceBytes(C.cast(ptr, C.c_void_p).value, nbytes), device="cuda").cpu().numpy()
+        return raw.view(dtype)
+
+    n, nlbi = int(cs.n_objects), int(cs.n_lbi)
+    return SimpleNamespace(
+        status_ga=pull(cs.status_ga, n, np.uint32), status_r53=pull(cs.status_r53, n, np.uint32), derived=pull(cs.derived, n, np.uint32),
+        ops=pull(cs.ops, cs.n_ops, abi.OP_DTYPE), section_begin=np.array(list(cs.section_begin), dtype=np.uint64),
+        tok_code=pull(cs.tok_code, nlbi, np.uint8), tok_name=pull(cs.tok_name, nlbi, np.uint64), tok_region=pull(cs.tok_region, nlbi, np.uint64),
+        dport_begin=pull(cs.dport_begin, n + 1, np.uint32), dports=pull(cs.dports, cs.n_dports, np.int32))
+
+
+def dump_outputs(cs, out_dir, max_values: int = DUMP_VALUES_MAX) -> dict:
+    """Write the change set `cs` (numpy arrays named as in abi.ChangeSet) as float64 `out_dir/<name>.npy`, every value exact:
+    ops as (n_ops, 6) rows of head, obj, sub, a0, a1, a2; the gar_str columns tok_name / tok_region as (n_lbi, 2) rows of slab
+    offset, length.  An array with more than `max_values` values keeps a sample of its rows: the same ascending row indices for
+    the same row count (fixed seed), so two runs on the same inputs are compared row for row.  `counts` holds the full sizes
+    (objects, ops, lbIngress hostnames, derived ports).  Returns {name: rows written}."""
+    import numpy as np
+    str_cols = lambda v: np.stack([v & np.uint64((1 << 40) - 1), v >> np.uint64(40)], axis=1)
+    arrays = {
+        "status_ga": cs.status_ga, "status_r53": cs.status_r53, "derived": cs.derived,
+        "ops": np.stack([cs.ops[f] for f in cs.ops.dtype.names], axis=1),
+        "section_begin": cs.section_begin, "tok_code": cs.tok_code, "tok_name": str_cols(cs.tok_name), "tok_region": str_cols(cs.tok_region),
+        "dport_begin": cs.dport_begin, "dports": cs.dports,
+        "counts": np.array([len(cs.status_ga), len(cs.ops), len(cs.tok_code), len(cs.dports)]),
+    }
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    written, total = {}, 0
+    for name, a in arrays.items():
+        rows = max(1, max_values // max(1, int(np.prod(a.shape[1:]))))
+        if len(a) > rows:
+            a = a[np.sort(np.random.default_rng(DUMP_SEED).choice(len(a), rows, replace=False))]
+        a = a.astype(np.float64)
+        total += a.nbytes
+        if total > DUMP_BYTES_MAX:
+            raise ValueError(f"--dump-outputs: more than {DUMP_BYTES_MAX >> 20} MB of outputs")
+        np.save(out_dir / f"{name}.npy", a)
+        written[name] = len(a)
+    return written
+
+
 TAG_OWNER_KEY, TAG_THOST_KEY = b"aws-global-accelerator-owner", b"aws-global-accelerator-target-hostname"
 TAG_MANAGED_KEY, TAG_CLUSTER_KEY = b"aws-global-accelerator-controller-managed", b"aws-global-accelerator-cluster"
 ANN_R53_KEY = b"aws-global-accelerator-controller.h3poteto.dev/route53-hostname"
@@ -558,7 +623,14 @@ def main():
                     help="sharded mode data path: p2p = pack kernels store straight into the other GPUs' receive arenas (CUDA IPC peer memory); "
                          "nccl = pack into a send buffer, torch.distributed all_to_all_single, unpack")
     ap.add_argument("--no-single", action="store_true", help="sharded: skip the single-GPU run of the same cluster (no checksum comparison)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the change set of the last timed step (rank 0) as DIR/<name>.npy, float64, "
+                         "at most 64 MB (large arrays as a fixed-seed sample of their rows; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "garecon" or args.mode != "replicas"):
+        ap.error("--dump-outputs writes the change set of the replicas step of this repo's engine (--impl garecon --mode replicas)")
     args.warmup = max(args.warmup, 3) if args.impl == "garecon" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -628,6 +700,8 @@ def main():
     barrier()
     t1 = time.perf_counter()
     dt_dev = max_over_ranks(t1 - t0 - t_flush)
+    if args.dump_outputs and rank == 0:  # before the e2e arm reloads the engine, which ends the device pointers of `cs`
+        dump_outputs(device_changeset(torch, cs), args.dump_outputs)
     b_alg = eng.algorithmic_bytes(cs)
     n_ops = int(cs.n_ops)
     n_pairs = eng.counters().get("r53_pairs", 0)

@@ -62,3 +62,38 @@ def test_byte_models_identify_keys_by_their_bytes(garecon):
     # the 300-byte decoy value is not part of what digest_accelerators must read: 5 x (4 + 18 + 70 + 7) system tag value bytes are
     sys_bytes = 5 * (len("true") + len("service/default/s0") + 70 + len("default"))
     assert big < sys_bytes + 5 * 300 + 16 * a.n_tags + 5 * 200
+
+
+def test_dump_outputs_is_exact_and_sampled_the_same_way_every_time(garecon, oracle, tmp_path):
+    """bench.py --dump-outputs: every change-set array as exact float64 (ops as rows of six fields, string references as offset and
+    length); above the size cap a sample of rows that depends only on the row count."""
+    import numpy as np
+    import randmodel
+    sys.path.insert(0, str(REPO))
+    bench = __import__("bench")
+    cs = oracle.diff(garecon.pack(*randmodel.make(3, n_objects=200)), "default", mode=1)
+    assert len(cs.ops) > 40 and len(cs.tok_name) > 40
+    rows = bench.dump_outputs(cs, tmp_path / "full")
+    load = lambda d, k: np.load(tmp_path / d / f"{k}.npy")
+    assert sorted(rows) == sorted(list(cs.ARRAYS) + ["counts"])
+    for k in cs.ARRAYS:
+        assert load("full", k).dtype == np.float64
+    assert (load("full", "status_ga") == cs.status_ga).all() and (load("full", "dports") == cs.dports).all()
+    assert (load("full", "ops").astype(np.uint32) == np.stack([cs.ops[f] for f in ("head", "obj", "sub", "a0", "a1", "a2")], axis=1)).all()
+    name = load("full", "tok_name").astype(np.uint64)
+    assert ((name[:, 1] << np.uint64(40)) | name[:, 0] == cs.tok_name).all()
+    assert load("full", "counts").tolist() == [200, len(cs.ops), len(cs.tok_code), len(cs.dports)]
+    for d in ("a", "b"):
+        rows = bench.dump_outputs(cs, tmp_path / d, max_values=24)
+    assert rows["status_ga"] == 24 and rows["ops"] == 4 and rows["tok_name"] == 12 and rows["section_begin"] == 5
+    for k in rows:
+        assert np.array_equal(load("a", k), load("b", k))
+    full_ops, ops = load("full", "ops"), load("a", "ops")
+    at = [next(i for i in range(len(full_ops)) if (full_ops[i] == r).all()) for r in ops]
+    assert at == sorted(at)
+
+
+def test_bench_rejects_zero_steps_and_dumps_it_cannot_make():
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "x"], ["--mode", "sharded", "--dump-outputs", "x"]):
+        out = subprocess.run([sys.executable, str(REPO / "bench.py"), *extra], capture_output=True, text=True, timeout=120, cwd=str(REPO))
+        assert out.returncode == 2 and "error" in out.stderr, extra
