@@ -19,7 +19,6 @@
 #include <thread>
 #include <string>
 #include <vector>
-#include <type_traits>
 #include <utility>
 
 #include "gar_pipeline.h"
@@ -41,8 +40,9 @@ __global__ void __launch_bounds__(256, MINB) k_for_each_warp(const __grid_consta
   u32 i = blockIdx.x * blockDim.x + threadIdx.x;
   f(i, i < n);
 }
-// ---- TMA-staged row passes (gar_pipeline.h "Staged"): one bulk copy (cp.async.bulk, completion on an mbarrier) brings the
-// block's string window(s) into shared memory; the row logic then reads shared memory instead of issuing its own global loads.
+// tokenise_hostnames, staged (gar_pipeline.h FTokenise): with column-major slabs the hostnames of a block's 256 consecutive rows
+// are ONE contiguous byte range.  One bulk copy (cp.async.bulk, completion on an mbarrier) brings it into shared memory and the
+// rows are tokenised from there; a string outside the staged window (other layouts, a wider window) is read from the slab.
 __device__ __forceinline__ u32 smem_addr(const void *p) { return (u32)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(u64 *bar, u32 count) {
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_addr(bar)), "r"(count));
@@ -62,58 +62,38 @@ __device__ __forceinline__ void mbar_wait(u64 *bar, u32 parity) {
     asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }" : "=r"(done) : "r"(smem_addr(bar)), "r"(parity) : "memory");
   } while (!done);
 }
-struct StagedView {
-  const u8 *smem[2];
-  const u8 *slab[2];
-  u64 lo[2], hi[2];  // staged slab byte range per window (hi includes 16 readable bytes of slack for the 8-byte unaligned loads)
-  __device__ __forceinline__ Str operator()(int c, gar_str r) const {
-    const u64 o = GAR_STR_OFF(r), n = GAR_STR_LEN(r);
-    if (o >= lo[c] && o + n + 16 <= hi[c]) return Str{smem[c] + (o - lo[c]), (u32)n};
-    return Str{slab[c] + o, (u32)n};
-  }
-};
-template <class F>
-__global__ void __launch_bounds__(256) k_for_each_staged(const __grid_constant__ F f, u32 n) {
-  constexpr u32 STAGE_BYTES = F::kStageBytes;  // per window
-  __shared__ alignas(128) u8 buf[F::kStageCols][STAGE_BYTES];
+constexpr u32 TOK_STAGE_BYTES = 24 * 1024;  // 256 lbIngress hostnames of ~70 bytes
+__global__ void __launch_bounds__(256) k_tokenise_staged(const __grid_constant__ FTokenise f, u32 n) {
+  __shared__ alignas(128) u8 buf[TOK_STAGE_BYTES];
   __shared__ alignas(8) u64 bar;
-  __shared__ u32 s_bytes[2];
-  __shared__ u64 s_lo[2];
+  __shared__ u64 s_lo;
+  __shared__ u32 s_bytes;
   const u32 r0 = blockIdx.x * blockDim.x, r1 = min(r0 + blockDim.x, n);
+  const u8 *slab = f.T.o.slab;
   if (threadIdx.x == 0) {
     mbar_init(&bar, 1);
-    u32 total = 0;
-    for (int c = 0; c < F::kStageCols; c++) {
-      u64 lo = 0, hi = 0;
-      u32 bytes = 0;
-      const u8 *slab = f.stage_slab(c);
-      if (f.stage_window(c, r0, r1, &lo, &hi) && hi > lo && (((uintptr_t)slab) & 15) == 0) {
-        lo &= ~(u64)15;
-        u64 span = ((hi - lo + 15) & ~(u64)15) + 16;  // + slack for over-reads; slabs carry GAR_SLAB_PAD readable bytes behind their end
-        if (span > STAGE_BYTES) span = STAGE_BYTES;   // a wider window (other layouts): the strings beyond it fall back to the slab
-        bytes = (u32)span;
-      }
-      s_lo[c] = lo;
-      s_bytes[c] = bytes;
-      total += bytes;
+    const gar_str a = f.T.o.lbi_hostname[r0], b = f.T.o.lbi_hostname[r1 - 1];
+    u64 lo = GAR_STR_OFF(a);
+    const u64 hi = GAR_STR_OFF(b) + GAR_STR_LEN(b);
+    u32 bytes = 0;
+    if (hi > lo && (((uintptr_t)slab) & 15) == 0) {
+      lo &= ~(u64)15;
+      const u64 span = ((hi - lo + 15) & ~(u64)15) + 16;  // + slack for over-reads; slabs carry GAR_SLAB_PAD readable bytes behind their end
+      bytes = (u32)(span < TOK_STAGE_BYTES ? span : TOK_STAGE_BYTES);
     }
-    mbar_expect_tx(&bar, total);
-    for (int c = 0; c < F::kStageCols; c++)
-      if (s_bytes[c]) tma_bulk_g2s(buf[c], f.stage_slab(c) + s_lo[c], s_bytes[c], &bar);
+    s_lo = lo;
+    s_bytes = bytes;
+    mbar_expect_tx(&bar, bytes);
+    if (bytes) tma_bulk_g2s(buf, slab + lo, bytes, &bar);
   }
   __syncthreads();
-  StagedView view;
-#pragma unroll
-  for (int c = 0; c < 2; c++) {
-    const bool on = c < F::kStageCols;
-    view.smem[c] = on ? buf[c < F::kStageCols ? c : 0] : nullptr;
-    view.slab[c] = on ? f.stage_slab(c) : nullptr;
-    view.lo[c] = on ? s_lo[c] : 1;
-    view.hi[c] = on ? s_lo[c] + s_bytes[c] : 0;
-  }
   mbar_wait(&bar, 0);
   const u32 i = r0 + threadIdx.x;
-  if (i < n) f.run(i, view);
+  if (i >= n) return;
+  const gar_str r = f.T.o.lbi_hostname[i];
+  const u64 o = GAR_STR_OFF(r), len = GAR_STR_LEN(r);
+  const bool staged = o >= s_lo && o + len + 16 <= s_lo + s_bytes;  // the 8-byte unaligned loads read up to 16 bytes past the end
+  tokenise_hostname_at(f.T, f.W, i, Str{staged ? buf + (o - s_lo) : slab + o, (u32)len});
 }
 
 // Count on the device (an intermediate relation whose size the host never learns mid-diff): one element per thread over the
@@ -452,52 +432,6 @@ struct StateError {
 
 static std::string g_create_error = "";
 
-// Sharded-mode pack, shared-memory variant (gar_shard.h FShPackRows; optional, GAR_PACK_TMA=1): one thread per selected row.  The
-// 256 rows of a block own one contiguous byte range of their destination's slab, so the block assembles it in shared memory and
-// one thread writes it with a bulk store (cp.async.bulk.global.shared::cta).  Blocks that straddle two destinations or exceed
-// the tile store directly.  Kept for the record: it lost against plain per-thread stores both locally and over NVLink.
-constexpr u32 PACK_TILE = 40 * 1024;
-__device__ __forceinline__ void bulk_s2g(void *dst, const void *src, u32 bytes) {
-  asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst), "r"(smem_addr(src)), "r"(bytes) : "memory");
-}
-__global__ void __launch_bounds__(256) k_shard_pack_rows(const __grid_constant__ FShPackRows f, u32 m) {
-  __shared__ alignas(128) u8 tile[PACK_TILE + 16];
-  __shared__ u32 s_staged, s_lo, s_bytes, s_d;
-  const u32 j0 = blockIdx.x * blockDim.x, j1 = min(j0 + blockDim.x, m), j = j0 + threadIdx.x;
-  if (threadIdx.x == 0) {
-    const u32 d0 = dest_of(j0, f.P.row_off, f.G), d1 = dest_of(j1 - 1, f.P.row_off, f.G);
-    const u32 lo = f.P.slab_scan[j0], hi = f.P.slab_scan[j1];
-    s_staged = f.S.n_str && d0 == d1 && hi > lo && hi - lo <= PACK_TILE;
-    s_lo = lo;
-    s_bytes = hi - lo;
-    s_d = d0;
-  }
-  __syncthreads();
-  if (!s_staged) {
-    if (j < m) f(j);
-    return;
-  }
-  const u32 d = s_d;
-  u8 *dst = f.D.base[d] + f.D.lay[d].slab + (s_lo - f.P.slab_scan[f.P.row_off[d]]);  // 8-byte aligned
-  u8 *t = tile + ((uintptr_t)dst & 15);                                               // same phase inside a 16-byte line as dst
-  if (j < m) f.row(j, t, s_lo);
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // the tile was written through the generic proxy, the bulk store reads it through the async one
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    const u32 bytes = s_bytes;                                  // multiple of 8
-    u32 head = ((uintptr_t)dst & 15) ? 8u : 0u;
-    if (head > bytes) head = bytes;
-    const u32 body = (bytes - head) & ~15u, tail = bytes - head - body;
-    if (head) *(u64 *)dst = *(const u64 *)t;
-    if (tail) *(u64 *)(dst + head + body) = *(const u64 *)(t + head + body);
-    if (body) {
-      bulk_s2g(dst + head, t + head, body);
-      asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-      asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");  // the tile must stay until it has been read
-    }
-  }
-}
-
 // Peer push (sharded mode, gar_shard_pack_peers): finished level groups of the staged blobs go to the other GPUs' receive arenas
 // over NVLink as 16-byte coalesced stores, one grid row per destination.  Runs on a high-priority stream beside the pack
 // kernels of the later levels.  (Measured at 8 GPUs, 2.6 GB to 7 peers per rank: copy engines 340 GB/s aggregate, last byte at
@@ -568,15 +502,11 @@ struct gar_engine {
   u8 *peer_ptr[2][GAR_SHARD_MAX_RANKS] = {};
   PeerHandle peer_seen[2][GAR_SHARD_MAX_RANKS] = {};
   bool peer_mapped[2][GAR_SHARD_MAX_RANKS] = {};
-  // staged transfer: the blobs for the other ranks are packed into `peer_stage` and moved by the copy engines, one stream per
-  // destination, level group by level group while the later levels still pack (GAR_PEER_DIRECT=1: the pack kernels store
-  // straight into the mapped arenas instead — one step, but 8-byte scattered stores over NVLink: 138 GB/s at 8 GPUs)
+  // staged transfer: the blobs for the other ranks are packed into `peer_stage` and pushed to their arenas by k_peer_push,
+  // level group by level group while the later levels still pack
   DBuf peer_stage;
-  cudaStream_t peer_copy_stream[GAR_SHARD_MAX_RANKS] = {};
   cudaStream_t peer_push_stream = nullptr;  // high priority: its blocks are placed before the pack kernels' next ones
-  bool peer_ce = false;                     // GAR_PEER_CE=1: move the staged blobs with cudaMemcpyAsync (copy engines) instead of k_peer_push
   std::vector<cudaEvent_t> peer_ev;
-  bool peer_direct = false;
   void peers_close() {
     for (int r = 0; r < 2; r++)
       for (int k = 0; k < GAR_SHARD_MAX_RANKS; k++) {
@@ -656,22 +586,10 @@ struct gar_engine {
   }
 
   // ---- Backend interface (gar_pipeline.h)
-  // GAR_PACK_TMA=1: the sharded pack assembles each block's slab range in shared memory and bulk-stores it (k_shard_pack_rows).
-  // Measured on the B200 (profiles/r02_pack_tma_ab.json): 10 % slower than per-thread stores into local memory (5.54 vs 5.02 ms,
-  // 2*10^6 objects) and 2.4x slower straight into peer arenas over NVLink (16.6 vs 6.8 ms per round-1 pack at 8 GPUs) — off.
-  bool pack_tma = false;
   template <class F>
   void for_each(const char *name, u32 n, const F &f) {
     if (!n) return;
     stage_begin(name);
-    if constexpr (std::is_same<F, FShPackRows>::value) {
-      if (pack_tma) {
-        k_shard_pack_rows<<<(n + 255) / 256, 256, 0, stream>>>(f, n);
-        launches++;
-        stage_end();
-        return;
-      }
-    }
     k_for_each<F><<<(n + 255) / 256, 256, 0, stream>>>(f, n);
     launches++;
     stage_end();
@@ -692,7 +610,6 @@ struct gar_engine {
   // so its first diff starts with buffers that fit (no grow-and-rerun on every load)
   u32 hint_dport_cap = 0, hint_pair_cap = 0;
   u64 hint_ops_cap = 0;
-  bool use_graphs = true;  // environment GAR_NO_GRAPH=1 turns it off
   cudaGraphExec_t graph_exec = nullptr;
   u64 graph_sig = 0, seen_sig = 0;
   u32 graph_launches = 0, capture_launch0 = 0;
@@ -703,7 +620,7 @@ struct gar_engine {
     graph_sig = seen_sig = 0;
   }
   int graph_begin(u64 sig) {
-    if (!use_graphs || timing) return 0;
+    if (timing) return 0;
     if (graph_exec && graph_sig == sig) {
       CK(cudaGraphLaunch(graph_exec, stream));
       launches += graph_launches;
@@ -736,15 +653,10 @@ struct gar_engine {
     graph_launches = launches - capture_launch0;
     CK(cudaGraphLaunch(graph_exec, stream));
   }
-  // environment GAR_NO_TMA=1: every staged row pass in its direct-load form; GAR_TMA_ALL=1: every one staged (A/B measurements).
-  // Default: each pass in the form that measured faster on the B200 (F::kStageByDefault).
-  bool staged_passes = true, staged_all = false;
-  template <class F>
-  void for_each_staged(const char *name, u32 n, const F &f) {
+  void for_each_staged(const char *name, u32 n, const FTokenise &f) {
     if (!n) return;
-    if (!staged_passes || !(F::kStageByDefault || staged_all)) return for_each(name, n, f);
     stage_begin(name);
-    k_for_each_staged<F><<<(n + 255) / 256, 256, 0, stream>>>(f, n);
+    k_tokenise_staged<<<(n + 255) / 256, 256, 0, stream>>>(f, n);
     launches++;
     stage_end();
   }
@@ -1294,12 +1206,6 @@ int gar_engine_create(const gar_config *cfg, gar_engine **out) {
   e->cluster = cfg->cluster_name ? cfg->cluster_name : "";
   e->timing = (cfg->flags & GAR_FLAG_STAGE_TIMING) != 0;
   e->reprepare = (cfg->flags & GAR_FLAG_REPREPARE) != 0;
-  if (const char *nt = getenv("GAR_NO_TMA")) e->staged_passes = nt[0] != '1';
-  if (const char *ta = getenv("GAR_TMA_ALL")) e->staged_all = ta[0] == '1';
-  if (const char *ng = getenv("GAR_NO_GRAPH")) e->use_graphs = ng[0] != '1';
-  if (const char *pd = getenv("GAR_PEER_DIRECT")) e->peer_direct = pd[0] == '1';
-  if (const char *pc = getenv("GAR_PEER_CE")) e->peer_ce = pc[0] == '1';
-  if (const char *pt = getenv("GAR_PACK_TMA")) e->pack_tma = pt[0] == '1';
   e->no_orphans = (cfg->flags & GAR_FLAG_NO_ORPHANS) != 0;
   e->allow_empty_cache = (cfg->flags & GAR_FLAG_ALLOW_EMPTY_CACHE) != 0;
   try {
@@ -1331,8 +1237,6 @@ void gar_engine_destroy(gar_engine *e) {
   e->peers_close();
   for (auto &b : e->peer_arena) cudaFree(b.p);
   cudaFree(e->peer_stage.p);
-  for (auto &cs : e->peer_copy_stream)
-    if (cs) cudaStreamDestroy(cs);
   if (e->peer_push_stream) cudaStreamDestroy(e->peer_push_stream);
   for (auto ev : e->peer_ev) cudaEventDestroy(ev);
   for (auto &ar : e->arena)
@@ -1545,10 +1449,10 @@ int gar_shard_pack_peers(gar_engine *e, int round, const uint64_t *all_meta) {
       bases[d] = e->peer_ptr[r][d] + off;
     }
     u32 l0 = e->launches;
-    if (e->peer_direct || G == 1) {
+    if (G == 1) {
       e->sharder->pack_to(bases);
     } else {
-      // own blob: packed in place.  The others: packed into the local stage, then pushed by the copy engines
+      // own blob: packed in place.  The others: packed into the local stage, then pushed by k_peer_push
       u64 stage_off[GAR_SHARD_MAX_RANKS + 1] = {0};
       for (u32 d = 0; d < G; d++)
         stage_off[d + 1] = stage_off[d] + (d == me ? 0 : blob_bytes(all_meta + ((size_t)me * G + d) * GAR_SHARD_META_WORDS));
@@ -1566,23 +1470,14 @@ int gar_shard_pack_peers(gar_engine *e, int round, const uint64_t *all_meta) {
       for (u32 d = 0; d < G; d++) {
         peer_base[d] = bases[d];
         if (d != me) bases[d] = (u8 *)st.p + stage_off[d];
-        if (e->peer_ce && d != me && !e->peer_copy_stream[d]) CK(cudaStreamCreateWithFlags(&e->peer_copy_stream[d], cudaStreamNonBlocking));
       }
-      if (!e->peer_ce && !e->peer_push_stream) {
+      if (!e->peer_push_stream) {
         int lo = 0, hi = 0;
         CK(cudaDeviceGetStreamPriorityRange(&lo, &hi));
         CK(cudaStreamCreateWithPriority(&e->peer_push_stream, cudaStreamNonBlocking, hi));
       }
       u64 sent[GAR_SHARD_MAX_RANKS] = {0};
       size_t ev_used = 0;
-      // GAR_PEER_TRACE=1: where the time of this call goes (stderr): pack kernels, first byte on the wire, last byte per destination
-      static const bool trace = getenv("GAR_PEER_TRACE") && getenv("GAR_PEER_TRACE")[0] == '1';
-      cudaEvent_t tr_begin = nullptr, tr_pack_end = nullptr, tr_first[GAR_SHARD_MAX_RANKS] = {}, tr_last[GAR_SHARD_MAX_RANKS] = {};
-      if (trace) {
-        CK(cudaEventCreate(&tr_begin));
-        CK(cudaEventCreate(&tr_pack_end));
-        CK(cudaEventRecord(tr_begin, e->stream));
-      }
       const u64 kGroupBytes = 48ull << 20;  // start a transfer once this much (over all destinations) is packed
       e->sharder->pack_to(bases, [&](int lvl, const u64 *end) {
         u64 pending = 0;
@@ -1596,71 +1491,22 @@ int gar_shard_pack_peers(gar_engine *e, int round, const uint64_t *all_meta) {
         }
         cudaEvent_t ev = e->peer_ev[ev_used++];
         CK(cudaEventRecord(ev, e->stream));
-        if (!e->peer_ce) {
-          PushDesc pd{};
-          u32 cnt = 0;
-          for (u32 k = 1; k < G; k++) {  // rank r starts with r+1: no destination is everybody's first
-            u32 d = (me + k) % G;
-            if (end[d] == sent[d]) continue;
-            pd.src[cnt] = (const uint4 *)(bases[d] + sent[d]);
-            pd.dst[cnt] = (uint4 *)(peer_base[d] + sent[d]);
-            pd.n16[cnt] = (end[d] - sent[d]) >> 4;  // blob sections are multiples of 16 bytes (sh_align)
-            sent[d] = end[d];
-            cnt++;
-          }
-          CK(cudaStreamWaitEvent(e->peer_push_stream, ev, 0));
-          if (trace && !tr_first[0]) {
-            CK(cudaEventCreate(&tr_first[0]));
-            CK(cudaEventRecord(tr_first[0], e->peer_push_stream));
-          }
-          k_peer_push<<<dim3(PUSH_BLOCKS, cnt), PUSH_THREADS, 0, e->peer_push_stream>>>(pd);
-          e->launches++;
-          return;
-        }
-        for (u32 k = 1; k < G; k++) {
+        PushDesc pd{};
+        u32 cnt = 0;
+        for (u32 k = 1; k < G; k++) {  // rank r starts with r+1: no destination is everybody's first
           u32 d = (me + k) % G;
           if (end[d] == sent[d]) continue;
-          CK(cudaStreamWaitEvent(e->peer_copy_stream[d], ev, 0));
-          if (trace && !tr_first[d]) {
-            CK(cudaEventCreate(&tr_first[d]));
-            CK(cudaEventRecord(tr_first[d], e->peer_copy_stream[d]));
-          }
-          CK(cudaMemcpyAsync(peer_base[d] + sent[d], bases[d] + sent[d], end[d] - sent[d], cudaMemcpyDefault, e->peer_copy_stream[d]));
+          pd.src[cnt] = (const uint4 *)(bases[d] + sent[d]);
+          pd.dst[cnt] = (uint4 *)(peer_base[d] + sent[d]);
+          pd.n16[cnt] = (end[d] - sent[d]) >> 4;  // blob sections are multiples of 16 bytes (sh_align)
           sent[d] = end[d];
+          cnt++;
         }
+        CK(cudaStreamWaitEvent(e->peer_push_stream, ev, 0));
+        k_peer_push<<<dim3(PUSH_BLOCKS, cnt), PUSH_THREADS, 0, e->peer_push_stream>>>(pd);
+        e->launches++;
       });
-      auto copy_stream = [&](u32 d) { return e->peer_ce ? e->peer_copy_stream[d] : e->peer_push_stream; };
-      if (trace) {
-        CK(cudaEventRecord(tr_pack_end, e->stream));
-        for (u32 d = 0; d < G; d++)
-          if (d != me) {
-            CK(cudaEventCreate(&tr_last[d]));
-            CK(cudaEventRecord(tr_last[d], copy_stream(d)));
-          }
-      }
-      for (u32 d = 0; d < G; d++)
-        if (d != me) CK(cudaStreamSynchronize(copy_stream(d)));
-      if (trace) {
-        CK(cudaStreamSynchronize(e->stream));
-        float pack_ms = 0;
-        CK(cudaEventElapsedTime(&pack_ms, tr_begin, tr_pack_end));
-        std::string line = "[peer trace] rank " + std::to_string(me) + " round " + std::to_string(round) + " groups " + std::to_string(ev_used) +
-                           " pack_end " + std::to_string(pack_ms) + " ms;";
-        for (u32 d = 0; d < G; d++)
-          if (d != me) {
-            float a = 0, b = 0;
-            cudaEvent_t first = e->peer_ce ? tr_first[d] : tr_first[0];
-            if (first) CK(cudaEventElapsedTime(&a, tr_begin, first));
-            CK(cudaEventElapsedTime(&b, tr_begin, tr_last[d]));
-            line += " ->" + std::to_string(d) + " " + std::to_string(sent[d] >> 20) + "MB first " + std::to_string(a).substr(0, 5) + " last " + std::to_string(b).substr(0, 5) + ";";
-            cudaEventDestroy(tr_last[d]);
-          }
-        for (auto &f : tr_first)
-          if (f) cudaEventDestroy(f);
-        fprintf(stderr, "%s\n", line.c_str());
-        cudaEventDestroy(tr_begin);
-        cudaEventDestroy(tr_pack_end);
-      }
+      CK(cudaStreamSynchronize(e->peer_push_stream));
     }
     e->shard_launches += e->launches - l0;
     CK(cudaStreamSynchronize(e->stream));  // the stores are performed: after the ranks' barrier every arena is complete

@@ -12,7 +12,8 @@
 //   void sort_pairs(u32 *keys, u32 *vals, u32 *keys_alt, u32 *vals_alt, u32 n, int bits);  // stable, result in keys/vals
 //   void fill32(u32 *p, u32 value, size_t n);
 //   void *ensure(int slot, size_t bytes);                                   // scratch buffer `slot`, at least `bytes`
-//   template <class F> void for_each_staged(const char *name, u32 n, const F &f);  // f(i), or f.run(i, view) with string windows staged on chip
+//   void for_each_staged(const char *name, u32 n, const FTokenise &f);      // f(i) for i in [0, n); the CUDA backend stages
+//                                                                           //   each block's hostnames in shared memory first
 //   template <class... Fs> void for_each_multi(const char *name, std::initializer_list<u32> ns, const Fs &...fs);  // ONE launch: fs[k](i), i < ns[k]
 //   template <class F> void for_each_dyn(const char *name, const u32 *n_dev, u32 cap, const F &f);       // f(i) for i < min(*n_dev, cap); the count
 //   template <class F> void for_each_warp_dyn(const char *name, const u32 *n_dev, u32 cap, const F &f);  //   lives on the device: no read-back
@@ -67,29 +68,12 @@ struct FClassify {
     derived_public[i] = dv & 0xFFu;
   }
 };
-// "Staged" row passes (CUDA backend: gar_engine.cu k_for_each_staged): with column-major slabs the strings of one column of a
-// block's consecutive rows are ONE contiguous byte range, so the block fetches that range with a single TMA bulk copy
-// (cp.async.bulk + mbarrier) into shared memory and parses from there.  A functor describes up to 2 windows:
-//   stage_window(c, r0, r1, &lo, &hi)  slab byte range [lo, hi) that holds column c's strings of rows [r0, r1)  (false: none)
-//   stage_slab(c)                      the slab the window lives in
-//   run(i, view)                       the row logic; view(c, ref) yields the string from shared memory when it lies inside the
-//                                      staged window and from the slab otherwise (other layouts simply fall back per string)
+// tokenise_hostnames is the one row pass whose strings are staged on chip (gar_engine.cu k_tokenise_staged): measured faster
+// on the B200 than direct loads (DESIGN.md §5); staging measured slower for prepare_records.
 struct FTokenise {
   DevTables T;
   Work W;
-  static constexpr int kStageCols = 1;
-  static constexpr u32 kStageBytes = 24 * 1024;  // 256 lbIngress hostnames of ~70 bytes
-  static constexpr bool kStageByDefault = true;
   GAR_HD void operator()(u32 i) const { tokenise_hostname(T, W, i); }
-  GAR_HD const u8 *stage_slab(int) const { return T.o.slab; }
-  GAR_HD bool stage_window(int, u32 r0, u32 r1, u64 *lo, u64 *hi) const {
-    gar_str a = T.o.lbi_hostname[r0], b = T.o.lbi_hostname[r1 - 1];
-    *lo = GAR_STR_OFF(a);
-    *hi = GAR_STR_OFF(b) + GAR_STR_LEN(b);
-    return true;
-  }
-  template <class View>
-  GAR_HD void run(u32 i, const View &view) const { tokenise_hostname_at(T, W, i, view(0, T.o.lbi_hostname[i])); }
 };
 struct FDigestAccel {
   DevTables T;
@@ -117,35 +101,11 @@ struct FExpand {
 // by its one thread: it goes on a list that FClassifyBigRecords works through with whole blocks.
 constexpr u32 REC_INLINE_VALUES = 32;   // more values than this: a whole block works on the record
 constexpr u32 REC_HUGE_VALUES = 4096;   // more than this: the whole grid does
-struct DirectView {  // the un-staged view: every string comes from its slab
-  const u8 *slab;
-  GAR_HD Str operator()(int, gar_str r) const { return mkstr(slab, r); }
-};
 struct FPrepareRecord {
   DevTables T;
   Work W;
   u32 *big, *huge;  // [0] = count, then record rows
-  static constexpr int kStageCols = 2;  // window 0: record names, window 1: the records' values
-  static constexpr u32 kStageBytes = 16 * 1024;  // 256 names of ~28 bytes; ~130 values of ~95 bytes
-  static constexpr bool kStageByDefault = false;  // measured on the B200 (profiles/r02_tma_ab.json): 0.297 ms staged vs 0.265 ms direct
-  GAR_HD const u8 *stage_slab(int) const { return T.a.slab; }
-  GAR_HD bool stage_window(int c, u32 r0, u32 r1, u64 *lo, u64 *hi) const {
-    if (c == 0) {
-      gar_str a = T.a.rec_name[r0], b = T.a.rec_name[r1 - 1];
-      *lo = GAR_STR_OFF(a);
-      *hi = GAR_STR_OFF(b) + GAR_STR_LEN(b);
-      return true;
-    }
-    u32 v0 = T.a.rec_val_begin[r0], v1 = T.a.rec_val_begin[r1];
-    if (v1 == v0) return false;
-    gar_str a = T.a.val_value[v0], b = T.a.val_value[v1 - 1];
-    *lo = GAR_STR_OFF(a);
-    *hi = GAR_STR_OFF(b) + GAR_STR_LEN(b);
-    return true;
-  }
-  GAR_HD void operator()(u32 r) const { run(r, DirectView{T.a.slab}); }
-  template <class View>
-  GAR_HD void run(u32 r, const View &view) const {
+  GAR_HD void operator()(u32 r) const {
     u32 lo = 0, hi = T.a.n_zones;
     while (hi - lo > 1) {
       u32 mid = (lo + hi) >> 1;
@@ -153,7 +113,7 @@ struct FPrepareRecord {
       else hi = mid;
     }
     W.rec_zone[r] = lo;
-    const Str nm = view(0, T.a.rec_name[r]);
+    const Str nm = mkstr(T.a.slab, T.a.rec_name[r]);
     const u64 nh = gar_hash(nm);
     W.rec_name_hash[r] = nh;
     W.rec_flags[r] = find_byte(nm, 0, '\\') < nm.n ? 1 : 0;
@@ -170,7 +130,7 @@ struct FPrepareRecord {
     }
     for (u32 v = v0; v < v1; v++) {
       W.val_rec[v] = r;
-      classify_value_at(T, W, v, view(1, T.a.val_value[v]));
+      classify_value(T, W, v);
     }
   }
 };
@@ -904,7 +864,7 @@ struct Pipeline {
       u32 *huge = (u32 *)be.ensure(S_SORT_VALS, 4 * (size_t)(nval / REC_HUGE_VALUES + 2));
       be.fill32(big, 0, 1);
       be.fill32(huge, 0, 1);
-      be.for_each_staged("prepare_records", nrec, FPrepareRecord{T, W, big, huge});
+      be.for_each("prepare_records", nrec, FPrepareRecord{T, W, big, huge});
       if (nval > REC_INLINE_VALUES) be.for_each("prepare_records", BIG_BLOCKS * 256, FClassifyBigRecords{T, W, big, huge});
     }
   }

@@ -349,7 +349,7 @@ GAR_HD u8 tokenise_str(Str h, u64 base, gar_str *name_out, gar_str *region_out) 
   *region_out = region;
   return code;
 }
-// h = the bytes of lbi_hostname[row] (in the slab, or staged in shared memory by the caller)
+// h = the bytes of lbi_hostname[row] (in the slab, or staged in shared memory by gar_engine.cu k_tokenise_staged)
 GAR_HD void tokenise_hostname_at(const DevTables &T, const Work &W, u32 row, Str h) {
   gar_str name, region;
   u8 code = tokenise_str(h, GAR_STR_OFF(T.o.lbi_hostname[row]), &name, &region);
@@ -455,10 +455,10 @@ GAR_HD void digest_accelerator(const DevTables &T, const Work &W, u32 a) {
 
 #define R53_HERITAGE "\"heritage=aws-global-accelerator-controller,cluster="
 
-// s = the bytes of val_value[v] (in the slab, or staged in shared memory by the caller)
-GAR_HD void classify_value_at(const DevTables &T, const Work &W, u32 v, Str s) {
+GAR_HD void classify_value(const DevTables &T, const Work &W, u32 v) {
   const gar_actual &A = T.a;
   gar_str ref = A.val_value[v];
+  const Str s = mkstr(A.slab, ref);
   u8 cls = VAL_NOT_OWNER;
   gar_str key = 0;
   const u32 hl = (u32)(sizeof(R53_HERITAGE) - 1);
@@ -480,7 +480,6 @@ GAR_HD void classify_value_at(const DevTables &T, const Work &W, u32 v, Str s) {
   W.val_key_hash[v] = vkh;
   if (cls) ix_count(W.hist[IX_VAL], vkh);
 }
-GAR_HD void classify_value(const DevTables &T, const Work &W, u32 v) { classify_value_at(T, W, v, mkstr(T.a.slab, T.a.val_value[v])); }
 
 // ------------------------------------------------------------------ index probes
 //

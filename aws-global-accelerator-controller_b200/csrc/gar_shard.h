@@ -409,13 +409,8 @@ struct FShPackRows {
   u32 G;
   PackDst D;
   u32 *any_long;  // device flag: some string was cut
-  // Optional CUDA variant (gar_engine.cu k_shard_pack_rows, GAR_PACK_TMA=1): a block's 256 consecutive rows own ONE contiguous
-  // byte range of the destination slab, so the block can assemble that range in shared memory and write it with one bulk store;
-  // row(j, tile, lo) puts row j's bytes at tile + (its slab position - lo).  tile == nullptr (the default path): straight to
-  // the destination, long strings cut.
-  static constexpr bool kBlockStagedStore = true;
-  GAR_HD void operator()(u32 j) const { row(j, nullptr, 0); }
-  GAR_HD void row(u32 j, u8 *tile, u32 tile_lo) const {
+  // straight to the destination, long strings cut (FShPackLong copies the rest)
+  GAR_HD void operator()(u32 j) const {
     u32 d = dest_of(j, P.row_off, G), k = j - P.row_off[d], p = P.sel[j];
     u8 *b = D.base[d];
     const LevelLayout &L = D.lay[d];
@@ -433,12 +428,8 @@ struct FShPackRows {
       u64 len = GAR_STR_LEN(ref[c]);
       ((gar_str *)(b + L.str[c]))[k] = GAR_STR(off, len);
       u32 words = sh_pad8((u32)len) >> 3;
-      if (tile) {
-        sh_copy_words((u64 *)(tile + (P.slab_scan[P.row_off[d]] + off - tile_lo)), src.slab + GAR_STR_OFF(ref[c]), words);
-      } else {
-        cut |= words > SH_LONG_WORDS;
-        sh_copy_words((u64 *)(b + L.slab + off), src.slab + GAR_STR_OFF(ref[c]), words > SH_LONG_WORDS ? SH_LONG_WORDS : words);
-      }
+      cut |= words > SH_LONG_WORDS;
+      sh_copy_words((u64 *)(b + L.slab + off), src.slab + GAR_STR_OFF(ref[c]), words > SH_LONG_WORDS ? SH_LONG_WORDS : words);
       off += (u64)words << 3;
     }
     if (cut) *any_long = 1;
@@ -859,9 +850,9 @@ struct Sharder {
     }
     pack_to(bases);
   }
-  // The pack kernels with one destination address per rank: bases[d] = where this rank's blob for rank d starts.  With peer
-  // memory mapped (gar_shard_pack_peers) these are addresses inside the OTHER GPUs' receive arenas: the rows travel over NVLink
-  // as the pack kernels store them — partitioning and transfer are one step, no staging buffer, no separate collective.
+  // The pack kernels with one destination address per rank: bases[d] = where this rank's blob for rank d starts: the send
+  // buffer, or with peer memory mapped (gar_shard_pack_peers) this rank's own receive arena for its own blob and a local stage
+  // for the others, which the engine then pushes to the other GPUs.
   // `level_done(l, end)` (optional) runs on the host after level l's kernels are queued; end[d] = bytes of destination d's blob
   // that are complete once those kernels have run — the engine uses it to start moving finished levels while later ones pack.
   template <class Done>

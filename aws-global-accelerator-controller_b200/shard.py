@@ -292,7 +292,7 @@ def add_checksums(parts) -> dict:
 
 class PeerExchange(DistExchange):
     """One process per GPU on one NVLink node: no collective on the data path.  Every rank maps the other GPUs' receive arenas
-    (CUDA IPC, include/garecon.h "Peer-memory exchange"); gar_shard_pack_peers packs and lets the copy engines push the blobs
+    (CUDA IPC, include/garecon.h "Peer-memory exchange"); gar_shard_pack_peers packs and a push kernel copies the blobs
     into the peers' arenas while later levels still pack.  torch.distributed moves one small all-gather per round (meta rows +
     arena handle, 0.4 KB per rank) and provides the barrier after the packs."""
 

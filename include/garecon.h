@@ -474,9 +474,8 @@ uint64_t gar_shard_blob_bytes(const uint64_t *meta_row);
    RECEIVE arenas of the other GPUs through CUDA IPC; gar_shard_pack_peers packs the rank's own blob in place and the others into a
    local stage from which a copy kernel on a high-priority stream pushes them into the peers' arenas over NVLink (16-byte coalesced
    stores), level group by level group while the later levels are still being packed (transfer and partitioning overlap).
-   Alternatives kept behind environment switches because they were measured and lost on 8 B200s: GAR_PEER_CE=1 (copy engines
-   instead of the copy kernel), GAR_PEER_DIRECT=1 (the pack kernels store straight into the mapped arenas: 8-byte scattered
-   stores over NVLink), GAR_PACK_TMA=1 (bulk stores from shared memory).  Per round:
+   On 8 B200s this beat copy engines, pack kernels storing straight into the mapped arenas, and bulk stores from shared memory
+   (DESIGN.md §6).  Per round:
 
      gar_shard_route(e, &shard, round, meta, send_bytes)
      all-gather the meta rows                                  -> all_meta[s][d] = row of source s for destination d
